@@ -51,6 +51,30 @@ MLP_NCU_DRAM_BYTES_PER_POSE = (3897.6e6 + 2588.9e6) / 151552   # profiles/r02_ml
 MLP_FLOP_PER_POSE = 4_714_240                                                     # SURVEY.md section 8a (a10)
 MLP_BYTES_PER_POSE = F * 4 + 3 * 4
 
+# --dump-outputs: outputs longer than DUMP_ROWS rows keep the same seeded sample of DUMP_ROWS rows, which holds the
+# 1M-row default run's dump to 27 MB
+DUMP_ROWS = 1 << 18
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each output as out_dir/<name>.npy.  With the same arguments the inputs and the sampled rows are the same
+    from run to run, so two builds of the project can be compared array for array."""
+    picked = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"{name}: {a.dtype} output")
+        if a.shape[0] > DUMP_ROWS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))]
+        picked[name] = a
+    total = sum(a.nbytes for a in picked.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes, more than {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in picked.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
 
 def load_artifacts():
     art = dict(np.load(os.path.join(ROOT, "tests", "golden", "shipped_artifacts.npz")))
@@ -333,8 +357,9 @@ def _pin_worker(n_workers):
         pass
 
 
-def bench_enlarged(spec, fitter_cls, torch, dist, world, rank, dev, num_sms, tf32_peak, peaks, with_cpu):
-    """One enlarged-core record: device-resident value, host-buffer e2e, tensor roofline (useful and issued), CPU port."""
+def bench_enlarged(spec, fitter_cls, torch, dist, world, rank, dev, num_sms, tf32_peak, peaks, with_cpu, outputs=None):
+    """One enlarged-core record: device-resident value, host-buffer e2e, tensor roofline (useful and issued), CPU port.
+    With `outputs` (a dict), the device-resident fit's last result goes there too."""
     from nlml_hpe_b200 import synthetic
     ranks = spec["ranks"]
     G, rws = enlarged_problem(ranks)
@@ -355,6 +380,8 @@ def bench_enlarged(spec, fitter_cls, torch, dist, world, rank, dev, num_sms, tf3
     ms, _ = time_steps(lambda: fit.fit(X, T_ITERS, LR, CLIP, out=P), spec["steps"], 0, torch, dist, world)
     launches = fit.launches - l0
     ms /= spec["steps"]
+    if outputs is not None:
+        outputs["enlarged_" + "x".join(map(str, ranks)) + "_fit"] = P.cpu().numpy()
     ms_e = time_host_steps(lambda: fit.fit_host(Xh.numpy(), T_ITERS, LR, CLIP, out=Ph), 1, 1, torch, dist, world)   # one warm-up: staging buffers
     fit.close()
     del X, Xh, P
@@ -522,6 +549,15 @@ def run_b200(args):
     tf32_peak = tf32_peak.value
     num_sms = torch.cuda.get_device_properties(dev).multi_processor_count
 
+    # --dump-outputs: what each timed device-resident call returned in its last step, copied to the host after timing
+    outputs = {} if args.dump_outputs else None
+    last = {}
+
+    def keep(name, fn):
+        def step():
+            last[name] = fn()
+        return step
+
     result = {}
     with ClockSampler(local) as clocks:
         # Tucker fit, device-resident
@@ -529,6 +565,8 @@ def run_b200(args):
         ms, wall = time_steps(lambda: fitter.fit(X, T_ITERS, LR, CLIP, out=P), steps, warmup, torch, dist, world)
         t_launches = (fitter.launches - l0) * steps // (steps + warmup)
         tucker_ms = ms / steps
+        if outputs is not None:
+            outputs["tucker_fit"] = P.cpu().numpy()
         # Tucker fit, host buffers through the C ABI (H2D + fit + D2H inside the timed region)
         e2e_steps = max(1, min(steps, args.e2e_steps))
         ms_e2e = time_host_steps(lambda: fitter.fit_host(X_host, T_ITERS, LR, CLIP, out=P_host), e2e_steps, 1, torch, dist, world)
@@ -538,6 +576,8 @@ def run_b200(args):
         ms_s, _ = time_steps(lambda: fitter.solve(X, out=P), steps, warmup, torch, dist, world)
         s_launches = (fitter.launches - l0) * steps // (steps + warmup)
         solve_ms = ms_s / steps
+        if outputs is not None:
+            outputs["tucker_solve"] = P.cpu().numpy()
         ms_se = time_host_steps(lambda: fitter.solve_host(X_host.numpy(), out=P_host), e2e_steps, 1, torch, dist, world)
         solve_e2e_ms = ms_se / e2e_steps
         _, ev = fitter.solve(X[:65536], return_evals=True)
@@ -547,11 +587,14 @@ def run_b200(args):
     with ClockSampler(local) as clocks2:
         l0 = model.launches
         model.predict(X[:1024])
-        ms_m, _ = time_steps(lambda: model.predict(X), steps, warmup, torch, dist, world)
+        ms_m, _ = time_steps(keep("mlp", lambda: model.predict(X)), steps, warmup, torch, dist, world)
         m_launches = (model.launches - l0) * steps // (steps + warmup)
         mlp_ms = ms_m / steps
         # the same forward fed RAW landmarks, IPD normalisation fused into the load stage (SURVEY.md section 8f row 3)
-        ms_lm, _ = time_steps(lambda: model.predict_landmarks(X), steps, warmup, torch, dist, world)
+        ms_lm, _ = time_steps(keep("mlp_landmarks", lambda: model.predict_landmarks(X)), steps, warmup, torch, dist, world)
+        if outputs is not None:
+            outputs.update((k, v.cpu().numpy()) for k, v in last.items())
+        last.clear()
         ms_me = time_host_steps(lambda: model.predict_host(X_host.numpy()), e2e_steps, 1, torch, dist, world)
         mlp_e2e_ms = ms_me / e2e_steps
     clk2 = clocks2.summary()
@@ -591,12 +634,14 @@ def run_b200(args):
             os.sched_setaffinity(0, all_cpus)
         for spec in ENLARGED:
             enlarged.append(bench_enlarged(spec, TuckerFitter, torch, dist, world, rank, dev, num_sms, tf32_peak, peaks,
-                                           with_cpu=(world == 1 and rank == 0 and not args.no_cpu_baseline)))
+                                           with_cpu=(world == 1 and rank == 0 and not args.no_cpu_baseline), outputs=outputs))
 
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     total = n * world
     tucker_pps = total / (tucker_ms * 1e-3)
     mlp_pps = total / (mlp_ms * 1e-3)
@@ -742,11 +787,21 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def _count(least):
+    def parse(s):
+        v = int(s)
+        if v < least:
+            raise argparse.ArgumentTypeError(f"{v} < {least}")
+        return v
+    return parse
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=_count(1), default=5,
+                    help="timed steps of the device-resident Tucker fit (headline), converged fit and Encoder+heads forwards")
+    ap.add_argument("--warmup", type=_count(0), default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--samples", type=int, default=1_000_000, help="feature vectors per GPU per step")
     ap.add_argument("--e2e-steps", type=int, default=3)
@@ -754,6 +809,10 @@ def main():
     ap.add_argument("--no-enlarged", action="store_true", help="skip the enlarged-core records (BASELINE.json configs[4])")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling records")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the rank to its GPU's NUMA-local CPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after timing, write what the device-resident Tucker fit, converged fit, Encoder+heads forward (on "
+                         "features and on raw landmarks) and enlarged-core fits returned in their last step as DIR/<name>.npy "
+                         f"(float32; a fixed seeded sample of {DUMP_ROWS} rows of longer outputs)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -33,7 +33,8 @@ def test_library_exports_every_declared_symbol(cuda_lib):
 def test_library_is_sm100a_only(cuda_lib):
     import subprocess
     from nlml_hpe_b200 import _build
-    out = subprocess.run(["cuobjdump", "-lelf", _build.LIB_PATH], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(_build._nvcc()), "cuobjdump")   # the toolkit that built the library, on PATH or not
+    out = subprocess.run([cuobjdump, "-lelf", _build.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
