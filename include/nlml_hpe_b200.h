@@ -95,6 +95,27 @@ int nlml_tucker_solve_host_f32(nlml_tucker_plan* plan, const float* X_host, int6
 int nlml_tucker_powell_f64(nlml_tucker_plan* plan, const float* X_dev, int64_t N, int64_t ldx, double* P_out_dev,
                            int64_t ldp, double* fun_out_dev, int32_t* nfev_out_dev, void* stream);
 
+/* The Tucker entry points on RAW MediaPipe landmarks: LM holds x,y,z of landmark i at columns 3i..3i+2 (column f =
+ * coordinate f % 3 of landmark f / 3), and every kernel's read of a row applies the normalisation of
+ * Read_Landmarks_and_Normalizing_using_IPD (/root/reference/helpers/FeatureExtractor.py:30-66, with the nose-tip reference
+ * point of :89-90 and the .float() of :105): subtract landmark 1, divide by ||landmark 33 - landmark 263|| (1e-6 when
+ * zero), in float64, rounded to float32 -- the same device code as nlml_mlp_forward_landmarks_f32.  Each call computes
+ * exactly what its feature twin computes on the normalised rows, bit for bit; kernel_hint, dispatch, asynchrony and the
+ * stride rules are the twin's.  The plan needs F >= 792 (landmark 263); NLML_E_INVALID otherwise.  Filtering the
+ * all-zero "no face" rows of the reference's callers stays the caller's job.  nlml_tucker_powell_landmarks_f64 equals the
+ * reference's FE.get_feature_vector(..., normalize=True) -> TD_Tester.Test chain bit for bit. */
+int nlml_tucker_fit_landmarks_f32(nlml_tucker_plan* plan, const float* LM_dev, int64_t N, int64_t ldx,
+                                  int iters, float lr, float clip, float* P_out_dev, int64_t ldp,
+                                  int kernel_hint, void* stream);
+int nlml_tucker_fit_landmarks_host_f32(nlml_tucker_plan* plan, const float* LM_host, int64_t N, int64_t ldx,
+                                       int iters, float lr, float clip, float* P_out_host, int64_t ldp);
+int nlml_tucker_solve_landmarks_f32(nlml_tucker_plan* plan, const float* LM_dev, int64_t N, int64_t ldx, int max_evals,
+                                    float* P_out_dev, int64_t ldp, int32_t* evals_out_dev, void* stream);
+int nlml_tucker_solve_landmarks_host_f32(nlml_tucker_plan* plan, const float* LM_host, int64_t N, int64_t ldx,
+                                         int max_evals, float* P_out_host, int64_t ldp);
+int nlml_tucker_powell_landmarks_f64(nlml_tucker_plan* plan, const float* LM_dev, int64_t N, int64_t ldx, double* P_out_dev,
+                                     int64_t ldp, double* fun_out_dev, int32_t* nfev_out_dev, void* stream);
+
 /* Test hook: phase A of the (5,3,3,3) kernels as the tensor-core GEMM the converged solve uses from 4096 samples on
  * (3xTF32 tcgen05, raw FP32 X tiles by TMA): q = W2 x, CTA-blocked, Q_out_dev [ceil(N/128)][136][128]
  * (q[r] of sample s at ((s / 128) * 136 + r) * 128 + s % 128).  Synchronous. */

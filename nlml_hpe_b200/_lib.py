@@ -17,6 +17,8 @@ EXPORTS = [
     "nlml_abi_version", "nlml_last_error",
     "nlml_tucker_plan_create", "nlml_tucker_plan_destroy", "nlml_tucker_fit_f32",
     "nlml_tucker_fit_host_f32", "nlml_tucker_solve_f32", "nlml_tucker_solve_host_f32", "nlml_tucker_launch_count",
+    "nlml_tucker_fit_landmarks_f32", "nlml_tucker_fit_landmarks_host_f32", "nlml_tucker_solve_landmarks_f32",
+    "nlml_tucker_solve_landmarks_host_f32", "nlml_tucker_powell_landmarks_f64",
     "nlml_tucker_powell_f64", "nlml_debug_powell_objective", "nlml_debug_project_tc", "nlml_cosine_fit_f64", "nlml_core_times_features_f32",
     "nlml_mlp_plan_create", "nlml_mlp_plan_destroy", "nlml_mlp_forward_f32",
     "nlml_mlp_forward_host_f32", "nlml_mlp_forward_landmarks_f32", "nlml_mlp_forward_landmarks_host_f32", "nlml_pose_postprocess_f64", "nlml_mlp_latent_f32", "nlml_mlp_launch_count", "nlml_mlp_set_path",
@@ -51,6 +53,11 @@ def load():
     lib.nlml_tucker_solve_f32.argtypes = [vp, vp, i64, i64, i32, vp, i64, vp, vp]
     lib.nlml_tucker_solve_host_f32.argtypes = [vp, vp, i64, i64, i32, vp, i64]
     lib.nlml_tucker_powell_f64.argtypes = [vp, vp, i64, i64, vp, i64, vp, vp, vp]
+    lib.nlml_tucker_fit_landmarks_f32.argtypes = lib.nlml_tucker_fit_f32.argtypes
+    lib.nlml_tucker_fit_landmarks_host_f32.argtypes = lib.nlml_tucker_fit_host_f32.argtypes
+    lib.nlml_tucker_solve_landmarks_f32.argtypes = lib.nlml_tucker_solve_f32.argtypes
+    lib.nlml_tucker_solve_landmarks_host_f32.argtypes = lib.nlml_tucker_solve_host_f32.argtypes
+    lib.nlml_tucker_powell_landmarks_f64.argtypes = lib.nlml_tucker_powell_f64.argtypes
     lib.nlml_debug_powell_objective.argtypes = [vp, vp, vp, i32, vp]
     lib.nlml_debug_project_tc.argtypes = [vp, vp, i64, i64, vp]
     lib.nlml_cosine_fit_f64.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, i32]

@@ -948,7 +948,8 @@ linear_tc2_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ L
 // IPD: the rows are RAW MediaPipe landmarks (x,y,z of landmark i at columns 3i..3i+2) and the translation /
 // scale normalisation of helpers/FeatureExtractor.py:30-66 (+ :89-90, :105) is applied on the way in: subtract the
 // nose tip (landmark 1), divide by the inter-pupillary distance ||lm33 - lm263|| (1e-6 when zero), in FLOAT64 as
-// the reference's Python floats, then round to float32 (`.float()`) -- so the encoder sees bit-identical inputs.
+// the reference's Python floats, then round to float32 (`.float()`) -- so the encoder sees bit-identical inputs
+// (ipd_row / ipd_map in common.cuh, shared with the Tucker kernels' raw-landmark loads).
 template <bool IPD>
 __global__ void __launch_bounds__(256) split_planes_kernel(const float* __restrict__ X, long long N, long long ldx, int K,
                                                           int Kp, int vec_ok, __half* __restrict__ Xhi,
@@ -971,15 +972,10 @@ __global__ void __launch_bounds__(256) split_planes_kernel(const float* __restri
         float f[4] = {v.x, v.y, v.z, v.w};
         if constexpr (IPD) {
             // the nine values every thread of the row needs come from L1 after the first touch
-            const double ref[3] = {(double)__ldg(src + 3), (double)__ldg(src + 4), (double)__ldg(src + 5)};
-            const double dx = (double)__ldg(src + 99) - (double)__ldg(src + 789);
-            const double dy = (double)__ldg(src + 100) - (double)__ldg(src + 790);
-            const double dz = (double)__ldg(src + 101) - (double)__ldg(src + 791);
-            double ipd = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
-            if (ipd == 0.0) ipd = 1e-6;
+            const IpdRow nr = ipd_row(src);
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                if (k + j < K) f[j] = __double2float_rn(__ddiv_rn(__dsub_rn((double)f[j], ref[(k + j) % 3]), ipd));
+                if (k + j < K) f[j] = ipd_map(f[j], nr, (k + j) % 3);
         }
         uint32_t h[2], l[2];
 #pragma unroll

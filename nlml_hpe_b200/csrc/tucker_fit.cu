@@ -51,6 +51,7 @@ struct TuckerArgs {
     int ri, ry, rp, rr;
     int nBCDp;
     int vec_ok;  // X rows and W2 rows are 16-byte aligned and F % 4 == 0
+    int ipd;     // X rows are raw landmarks: phase A reads them through the IPD normalisation (common.cuh)
 #ifdef NLML_TC_DBG
     int dbg;     // development build only (-DNLML_TC_DBG): tensor-core kernel 1 = no MMAs / waits, 2 = no TMEM consumption
 #endif
@@ -187,6 +188,10 @@ struct TpsCfg {
     static constexpr int TILE_FLOATS = FC * XSTR + FC * RPAD;
 
     static_assert(!QTMEM || TILE_FLOATS <= SCR_FLOATS, "phase-A tiles alias the scratch buffer in the TMEM variant");
+    // raw-landmark input: the (ref, ipd) of the pass's THREADS rows live in the scratch buffer during phase A (after the
+    // tiles in the TMEM variant)
+    static constexpr int IPD_OFF = QTMEM ? (TILE_FLOATS + 1) / 2 * 2 : 0;
+    static_assert(IPD_OFF * 4 + THREADS * sizeof(IpdRow) <= SCR_FLOATS * 4, "IPD constants fit the scratch buffer");
     static constexpr size_t SMEM_BYTES = sizeof(float) * (S_FLOATS + Q_FLOATS + SCR_FLOATS) + 16;
 };
 
@@ -249,6 +254,12 @@ __global__ void __launch_bounds__(THREADS, MINB) tucker_fit_tps_kernel(const __g
     float* qn_s = QTMEM ? scr_s : q_s + n * (C::R * THREADS);   // TMEM variant: tiles live in the scratch buffer
     xs = qn_s;
     ws = qn_s + C::FC * C::XSTR;
+    IpdRow* ipd_s = reinterpret_cast<IpdRow*>(scr_s + C::IPD_OFF);
+    if (a.ipd) {   // raw landmarks: each row's (ref, ipd) once per pass, applied to the staged tiles below
+        const long long row = s0 + n * THREADS + tid;
+        if (row < a.N) ipd_s[tid] = ipd_row(a.X + row * a.ldx);
+        __syncthreads();
+    }
     float acc[C::RPAD];
 #pragma unroll
     for (int r = 0; r < C::RPAD; ++r) acc[r] = 0.f;
@@ -274,6 +285,10 @@ __global__ void __launch_bounds__(THREADS, MINB) tucker_fit_tps_kernel(const __g
             ws[(4 * c4 + 3) * C::RPAD + r] = v.w;
         }
         __syncthreads();
+        if (a.ipd) {
+            ipd_tile(xs, C::XSTR, C::FC, THREADS, ipd_s, a.N - (s0 + n * THREADS), f0, F, tid, THREADS);
+            __syncthreads();
+        }
 #pragma unroll 4
         for (int f = 0; f < C::FC; ++f) {
             const float xv = xs[f * C::XSTR + tid];
@@ -419,7 +434,12 @@ __global__ void __launch_bounds__(THREADS) tucker_fit_cta_kernel(const __grid_co
 
     const long long s = blockIdx.x;
     const float* xrow = a.X + s * a.ldx;
-    for (int f = tid; f < F; f += THREADS) xb[f] = __ldg(xrow + f);
+    if (a.ipd) {   // raw landmarks: every thread derives the row's (ref, ipd) from the same nine L1-resident values
+        const IpdRow nr = ipd_row(xrow);
+        for (int f = tid; f < F; f += THREADS) xb[f] = ipd_map(__ldg(xrow + f), nr, f % 3);
+    } else {
+        for (int f = tid; f < F; f += THREADS) xb[f] = __ldg(xrow + f);
+    }
     for (int idx = tid; idx < 4 * kMaxPairs; idx += THREADS) {
         const int m = idx / kMaxPairs, k = idx % kMaxPairs;
         int i = 0, j = 0;
@@ -652,7 +672,12 @@ __global__ void __launch_bounds__(32 * WARPS) tucker_fit_wps_kernel(const __grid
     // ---- phase A: q = W2 x (warp-cooperative dot products, x staged in shared memory) ----
     if (live) {
         const float* xrow = a.X + s * a.ldx;
-        for (int f = lane; f < Fp; f += 32) xb[f] = f < F ? __ldg(xrow + f) : 0.f;
+        if (a.ipd) {   // raw landmarks: each lane derives the row's (ref, ipd); the pad columns stay zero
+            const IpdRow nr = ipd_row(xrow);
+            for (int f = lane; f < Fp; f += 32) xb[f] = f < F ? ipd_map(__ldg(xrow + f), nr, f % 3) : 0.f;
+        } else {
+            for (int f = lane; f < Fp; f += 32) xb[f] = f < F ? __ldg(xrow + f) : 0.f;
+        }
     }
     __syncwarp();
     if (live) {
@@ -926,6 +951,13 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
 #pragma unroll
             for (int r = 0; r < RH; ++r) acc[r] = __ldg(slab + r * 128);
         }
+        // raw landmarks: the 128 rows' (ref, ipd) once, in the gradient exchange buffer (unused until phase B)
+        IpdRow* ipd_s = reinterpret_cast<IpdRow*>(gx);
+        static_assert(C::THREADS * sizeof(IpdRow) <= C::NGX * C::THREADS * 4, "IPD constants fit the exchange buffer");
+        if (a.ipd && !a.Qpre) {
+            if (role == 0 && s0 + row < a.N) ipd_s[row] = ipd_row(a.X + (s0 + row) * a.ldx);
+            __syncthreads();
+        }
         for (int f0 = 0; f0 < (a.Qpre ? 0 : F); f0 += C::FC) {
             for (int idx = tid; idx < C::THREADS * (C::FC / 4); idx += 256) {
                 const int s = idx / (C::FC / 4), c4 = idx % (C::FC / 4);
@@ -947,6 +979,10 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
                 ws[(4 * c4 + 3) * C::RPAD + r] = v.w;
             }
             __syncthreads();
+            if (a.ipd) {
+                ipd_tile(xs, C::XSTR, C::FC, C::THREADS, ipd_s, a.N - s0, f0, F, tid, 256);
+                __syncthreads();
+            }
 #pragma unroll 4
             for (int f = 0; f < C::FC; ++f) {
                 const float xv = xs[f * C::XSTR + row];
@@ -1251,6 +1287,7 @@ struct PowellArgs {
     double* fun;          // [N] or null
     int* nfev;            // [N] or null
     int ri, ry, rp, rr, F;
+    int ipd;              // X rows are raw landmarks: x is staged through the IPD normalisation (common.cuh)
     int nleaf, nprog;
     short leaf_off[kPowellMaxLeaves], leaf_len[kPowellMaxLeaves];
     signed char prog[2 * kPowellMaxLeaves];   // postfix combine program of the pairwise tree: k >= 0 push leaf k, -1 add
@@ -1349,7 +1386,13 @@ __global__ void __launch_bounds__(kPowellThreads) tucker_powell_kernel(const __g
     double* result = leafsum + kPowellMaxLeaves;
     float* xs = reinterpret_cast<float*>(result + 2);
     const long long s = blockIdx.x;
-    for (int f = threadIdx.x; f < a.F; f += kPowellThreads) xs[f] = __ldg(a.X + s * a.ldx + f);
+    const float* xrow = a.X + s * a.ldx;
+    if (a.ipd) {   // raw landmarks: x becomes the float32 vector FE.get_feature_vector(..., normalize=True) returns
+        const IpdRow nr = ipd_row(xrow);
+        for (int f = threadIdx.x; f < a.F; f += kPowellThreads) xs[f] = ipd_map(__ldg(xrow + f), nr, f % 3);
+    } else {
+        for (int f = threadIdx.x; f < a.F; f += kPowellThreads) xs[f] = __ldg(xrow + f);
+    }
     __syncthreads();
     PowellCoopObjective obj{a, xs, e, racc, leafsum, result};
     const int NP = 3 + a.ri;
@@ -1434,6 +1477,9 @@ struct ProjArgs {
     int F, RPAD, num_kb;
     const uint8_t* wtiles;   // [num_kb][W_BYTES]
     float* Q;                // [tiles][RPAD][128]
+    int ipd;                 // X rows are raw landmarks: the converters apply the IPD normalisation before the split
+    const float* X;          // ... and read each row's (ref, ipd) from here (the tensor map's base, row pitch ldx floats)
+    long long ldx;
 };
 __device__ __forceinline__ uint64_t proj_desc_sw128(uint32_t smem_addr) {   // K-major, 128-byte swizzle, 8-row groups 1024 B apart
     uint64_t d = 0;
@@ -1518,7 +1564,13 @@ __global__ void __launch_bounds__(ProjCfg::THREADS, 1) tucker_project_tc_kernel(
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(64));
         const int r = tid - 128;
         int s = 0; uint32_t ph = 0;
-        for (long long t = blockIdx.x; t < tiles; t += gridDim.x)
+        for (long long t = blockIdx.x; t < tiles; t += gridDim.x) {
+            // raw landmarks: this row's (ref, ipd) once per tile (nine L2 hits), kept in registers across the k-blocks; rows
+            // past N are the tensor map's zero fill and stay zero
+            const long long grow = t * C::BM + r;
+            const bool map = a.ipd && grow < a.N;
+            IpdRow nr{};
+            if (map) nr = ipd_row(a.X + grow * a.ldx);
             for (int kb = 0; kb < a.num_kb; ++kb) {
                 ttc::mbar_wait(&full[s], ph);
                 uint8_t* xh = sm + (size_t)s * C::STAGE_BYTES + r * 128;
@@ -1527,8 +1579,10 @@ __global__ void __launch_bounds__(ProjCfg::THREADS, 1) tucker_project_tc_kernel(
                 for (int cc = 0; cc < 8; ++cc) {
                     // the swizzle permutes whole 16-byte chunks, so position-wise processing is enough; the threads of 8
                     // consecutive rows take different chunk positions at a time (rows are 128 B apart: all on the same banks otherwise)
+                    // (position c holds logical chunk c ^ (r & 7) = cc: features kb*32 + 4cc .. +3)
                     const int c = cc ^ (r & 7);
                     float4 v = *reinterpret_cast<float4*>(xh + 16 * c);
+                    if (map) v = ipd_map4(v, nr, kb * C::BK + 4 * cc, a.F);
                     float4 h, l;
                     ttc::split_tf32_bits(v.x, h.x, l.x); ttc::split_tf32_bits(v.y, h.y, l.y);
                     ttc::split_tf32_bits(v.z, h.z, l.z); ttc::split_tf32_bits(v.w, h.w, l.w);
@@ -1540,6 +1594,7 @@ __global__ void __launch_bounds__(ProjCfg::THREADS, 1) tucker_project_tc_kernel(
                 if (lane == 0) tgen::mbar_arrive(&conv[s]);
                 if (++s == C::STAGES) { s = 0; ph ^= 1u; }
             }
+        }
     } else {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(232));
         const int row = tid - 256;
@@ -1836,7 +1891,7 @@ int64_t gen_chunk(const nlml_tucker_plan* pl) {
     return std::min<int64_t>(waves, 8) * wave;
 }
 
-int launch_gen(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int iters, float lr, float clip, float* P,
+int launch_gen(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int ipd, int iters, float lr, float clip, float* P,
                int64_t ldp, int ws_slot, cudaStream_t st) {
     const int64_t chunk = gen_chunk(pl);
     const int64_t want = std::min<int64_t>(chunk, ceil_div(N, tgen::kSamples) * tgen::kSamples);
@@ -1866,7 +1921,7 @@ int launch_gen(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
         const float* x = X + s0 * ldx;
         const int vec_ok = (pl->F % 4 == 0) && (ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
         const unsigned ctas = (unsigned)ceil_div(n, tgen::kSamples);
-        tgen::tucker_project_kernel<<<dim3(ctas, (unsigned)ceil_div(pl->R, 64)), 256, 0, st>>>(x, n, ldx, pl->W2, pl->R, pl->F, vec_ok, pl->q_ws[ws_slot]);
+        tgen::tucker_project_kernel<<<dim3(ctas, (unsigned)ceil_div(pl->R, 64)), 256, ipd ? sizeof(IpdRow) * tgen::kSamples : 0, st>>>(x, n, ldx, pl->W2, pl->R, pl->F, vec_ok, pl->q_ws[ws_slot], ipd);
         a.P = P + s0 * ldp;
         a.N = n;
         if (int rc = dispatch_gen(a, ctas, st, false)) return rc;
@@ -1878,10 +1933,11 @@ int launch_gen(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
 }
 
 constexpr int64_t kProjMinRows = 4096;   // below this the consumer's own phase A is as fast (one partial wave)
-int project_tc(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, cudaStream_t st, const float** Qout,
+int project_tc(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int ipd, cudaStream_t st, const float** Qout,
                int64_t min_rows = kProjMinRows);
 
-int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int iters, float lr, float clip,
+// ipd: X holds raw landmarks; every phase A below reads it through the IPD normalisation (common.cuh)
+int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int ipd, int iters, float lr, float clip,
                float* P, int64_t ldp, int hint, cudaStream_t st, int ws_slot = 2, int64_t proj_min_rows = kProjMinRows) {
     if (N == 0) return 0;
     // run-time-rank tensor-core kernel: asked for, or the default for every rank set without compiled kernels
@@ -1890,11 +1946,12 @@ int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
     if (hint == 2 && !pl->cta_ok)
         return set_error(NLML_E_UNSUPPORTED, "core too large for the CTA-per-sample kernel's shared-memory working set");
     if (hint == 6 || (hint == 0 && !pl->fast && pl->gen_ok && (N >= 32 || !pl->cta_ok)))
-        return launch_gen(pl, X, N, ldx, iters, lr, clip, P, ldp, ws_slot, st);
+        return launch_gen(pl, X, N, ldx, ipd, iters, lr, clip, P, ldp, ws_slot, st);
     TuckerArgs a = pl->base;
     a.X = X;
     a.N = N;
     a.ldx = ldx;
+    a.ipd = ipd;
     a.P = P;
     a.ldp = ldp;
     a.T = iters;
@@ -1916,12 +1973,15 @@ int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
         return set_error(NLML_E_UNSUPPORTED, "thread/warp-per-sample kernels are built for ranks (5,3,3,3) only");
     if (use_tc) {
         // phase A (q = W2 x) as a 3xTF32 tcgen05 GEMM of its own when the layout allows TMA; the kernel then only copies its slab
-        if (int rc = project_tc(pl, X, N, ldx, st, &a.Qpre, proj_min_rows)) return rc;
+        if (int rc = project_tc(pl, X, N, ldx, ipd, st, &a.Qpre, proj_min_rows)) return rc;
         tucker_fit_tc_kernel<<<(unsigned)ceil_div(N, TcFitCfg::THREADS), 2 * TcFitCfg::THREADS, TcFitCfg::SMEM_BYTES, st>>>(a);
         if (a.Qpre) NLML_CUDA(cudaEventRecord(pl->q_pre_done, st));
     } else if (use_wps) {
         auto kern = tucker_fit_wps_kernel<5, 3, 3, 3, kWpsWarps>;
         const unsigned grid = (unsigned)ceil_div(N, kWpsWarps);
+        // the shared-memory limit is a property of the function, not of the plan: a plan with a smaller F created since
+        // may have lowered it (as for the Powell kernel, it is set at each launch)
+        NLML_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wps_smem_bytes(pl->F)));
         kern<<<grid, 32 * kWpsWarps, wps_smem_bytes(pl->F), st>>>(a);
     } else if (use_tps) {
         if (hint == 4) {
@@ -1933,6 +1993,7 @@ int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
         }
     } else {
         auto kern = tucker_fit_cta_kernel<kCtaThreads>;
+        NLML_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->cta_smem));   // as above
         kern<<<(unsigned)N, kCtaThreads, pl->cta_smem, st>>>(a, pl->st_in_smem ? 1 : 0);
     }
     NLML_CUDA(cudaGetLastError());
@@ -1945,7 +2006,7 @@ int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
 typedef CUresult (*EncodeTiledFnT)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-int project_tc(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, cudaStream_t st, const float** Qout, int64_t min_rows) {
+int project_tc(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int ipd, cudaStream_t st, const float** Qout, int64_t min_rows) {
     *Qout = nullptr;
     if (!pl->fast || !pl->proj_tiles || N < min_rows || (ldx % 4) != 0 || (reinterpret_cast<uintptr_t>(X) & 15) != 0) return 0;
     static EncodeTiledFnT encode = nullptr;
@@ -1977,6 +2038,7 @@ int project_tc(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, cud
     ProjArgs pa{};
     pa.N = N; pa.F = pl->F; pa.RPAD = 136; pa.num_kb = (pl->F + ProjCfg::BK - 1) / ProjCfg::BK;
     pa.wtiles = pl->proj_tiles; pa.Q = pl->q_pre;
+    pa.ipd = ipd; pa.X = X; pa.ldx = ldx;
     const unsigned grid = (unsigned)std::min<int64_t>(tiles, pl->num_sms);
     tucker_project_tc_kernel<<<grid, ProjCfg::THREADS, ProjCfg::SMEM_BYTES, st>>>(xmap, pa);
     NLML_CUDA(cudaGetLastError());
@@ -1986,7 +2048,7 @@ int project_tc(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, cud
 }
 
 // converged fit (SURVEY.md section 8f row 1): thread-per-sample kernel, phase B' = tucker_lm_solve
-int launch_solve(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int max_evals, float* P, int64_t ldp,
+int launch_solve(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int ipd, int max_evals, float* P, int64_t ldp,
                  int* evals, cudaStream_t st, int64_t proj_min_rows = kProjMinRows) {
     if (N == 0) return 0;
     if (!pl->fast) return set_error(NLML_E_UNSUPPORTED, "the converged solve is built for ranks (5,3,3,3) only");
@@ -1994,13 +2056,14 @@ int launch_solve(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, i
     a.X = X;
     a.N = N;
     a.ldx = ldx;
+    a.ipd = ipd;
     a.P = P;
     a.ldp = ldp;
     a.vec_ok = (pl->F % 4 == 0) && (ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
     a.lm = lm_default_options();
     if (max_evals > 0) a.lm.max_evals = max_evals;
     a.evals = evals;
-    if (int rc = project_tc(pl, X, N, ldx, st, &a.Qpre, proj_min_rows)) return rc;   // phase A as a tensor-core GEMM when the layout allows TMA
+    if (int rc = project_tc(pl, X, N, ldx, ipd, st, &a.Qpre, proj_min_rows)) return rc;   // phase A as a tensor-core GEMM when the layout allows TMA
     auto kern = tucker_fit_tps_kernel<5, 3, 3, 3, kTpsThreads, 1, kSolveMinBlocks, false, true>;
     kern<<<(unsigned)ceil_div(N, TpsDefault::SAMPLES), kTpsThreads, TpsDefault::SMEM_BYTES, st>>>(a);
     NLML_CUDA(cudaGetLastError());
@@ -2263,54 +2326,104 @@ extern "C" void nlml_tucker_plan_destroy(nlml_tucker_plan* pl) {
     delete pl;
 }
 
-extern "C" int nlml_tucker_fit_f32(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int iters,
-                                   float lr, float clip, float* P_out_dev, int64_t ldp, int kernel_hint,
-                                   void* stream) {
+namespace {
+// the raw-landmark entry points (ipd = 1) read landmarks 1, 33 and 263: columns 3..5, 99..101 and 789..791
+int check_landmark_plan(const nlml_tucker_plan* pl, int ipd) {
+    if (ipd && pl->F < 3 * 264)
+        return set_error(NLML_E_INVALID, "IPD normalisation needs x,y,z triples up to landmark 263 (F=%d)", pl->F);
+    return 0;
+}
+
+int fit_device(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int ipd, int iters, float lr, float clip,
+               float* P_out_dev, int64_t ldp, int kernel_hint, void* stream) {
     if (!pl || (N > 0 && (!X_dev || !P_out_dev))) return set_error(NLML_E_INVALID, "null pointer argument");
     if (N < 0 || ldx < pl->F || ldp < 3 + pl->ri || iters < 0)
         return set_error(NLML_E_INVALID, "bad sizes: N=%lld ldx=%lld (F=%d) ldp=%lld (need >= %d) iters=%d",
                          (long long)N, (long long)ldx, pl->F, (long long)ldp, 3 + pl->ri, iters);
     if (kernel_hint < 0 || kernel_hint > 6) return set_error(NLML_E_INVALID, "kernel_hint must be 0..6");
+    if (int rc = check_landmark_plan(pl, ipd)) return rc;
     DeviceGuard guard(pl->device);
-    return launch_fit(pl, X_dev, N, ldx, iters, lr, clip, P_out_dev, ldp, kernel_hint, (cudaStream_t)stream);
+    return launch_fit(pl, X_dev, N, ldx, ipd, iters, lr, clip, P_out_dev, ldp, kernel_hint, (cudaStream_t)stream);
 }
 
-extern "C" int nlml_tucker_fit_host_f32(nlml_tucker_plan* pl, const float* X_host, int64_t N, int64_t ldx,
-                                        int iters, float lr, float clip, float* P_out_host, int64_t ldp) {
+int fit_host(nlml_tucker_plan* pl, const float* X_host, int64_t N, int64_t ldx, int ipd, int iters, float lr, float clip,
+             float* P_out_host, int64_t ldp) {
     if (!pl || (N > 0 && (!X_host || !P_out_host))) return set_error(NLML_E_INVALID, "null pointer argument");
     if (N < 0 || ldx < pl->F || ldp < 3 + pl->ri || iters < 0) return set_error(NLML_E_INVALID, "bad sizes");
+    if (int rc = check_landmark_plan(pl, ipd)) return rc;
     DeviceGuard guard(pl->device);
     const int np = 3 + pl->ri;
     // every chunk runs the kernel the whole batch would get (the first chunks of the ramp are below the cross-over)
     const int hint = (pl->fast && N >= tc_crossover(pl)) ? 5 : 0;
     const int64_t proj_min = hint == 5 ? 1 : kProjMinRows;   // ... and the phase A the whole batch would get
     return host_pipeline(pl, X_host, N, ldx, P_out_host, ldp, [&](const float* x, int64_t n, float* p, cudaStream_t st, int slot) {
-        return launch_fit(pl, x, n, pl->F, iters, lr, clip, p, np, hint, st, slot, proj_min);
+        return launch_fit(pl, x, n, pl->F, ipd, iters, lr, clip, p, np, hint, st, slot, proj_min);
     });
 }
 
-extern "C" int nlml_tucker_solve_f32(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int max_evals,
-                                     float* P_out_dev, int64_t ldp, int32_t* evals_out_dev, void* stream) {
+int solve_device(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int ipd, int max_evals, float* P_out_dev,
+                 int64_t ldp, int32_t* evals_out_dev, void* stream) {
     if (!pl || (N > 0 && (!X_dev || !P_out_dev))) return set_error(NLML_E_INVALID, "null pointer argument");
     if (N < 0 || ldx < pl->F || ldp < 3 + pl->ri || max_evals < 0 || max_evals == 1)
         return set_error(NLML_E_INVALID, "bad sizes: N=%lld ldx=%lld (F=%d) ldp=%lld (need >= %d) max_evals=%d (0 = default, else >= 2)",
                          (long long)N, (long long)ldx, pl->F, (long long)ldp, 3 + pl->ri, max_evals);
+    if (int rc = check_landmark_plan(pl, ipd)) return rc;
     DeviceGuard guard(pl->device);
-    return launch_solve(pl, X_dev, N, ldx, max_evals, P_out_dev, ldp, evals_out_dev, (cudaStream_t)stream);
+    return launch_solve(pl, X_dev, N, ldx, ipd, max_evals, P_out_dev, ldp, evals_out_dev, (cudaStream_t)stream);
 }
 
-extern "C" int nlml_tucker_solve_host_f32(nlml_tucker_plan* pl, const float* X_host, int64_t N, int64_t ldx,
-                                          int max_evals, float* P_out_host, int64_t ldp) {
+int solve_host(nlml_tucker_plan* pl, const float* X_host, int64_t N, int64_t ldx, int ipd, int max_evals, float* P_out_host,
+               int64_t ldp) {
     if (!pl || (N > 0 && (!X_host || !P_out_host))) return set_error(NLML_E_INVALID, "null pointer argument");
     if (N < 0 || ldx < pl->F || ldp < 3 + pl->ri || max_evals < 0 || max_evals == 1) return set_error(NLML_E_INVALID, "bad sizes");
     if (!pl->fast) return set_error(NLML_E_UNSUPPORTED, "the converged solve is built for ranks (5,3,3,3) only");
+    if (int rc = check_landmark_plan(pl, ipd)) return rc;
     DeviceGuard guard(pl->device);
     const int np = 3 + pl->ri;
     // every chunk takes the phase A the whole batch would get (the last chunk of the ramp may be below the threshold)
     const int64_t proj_min = N >= kProjMinRows ? 1 : kProjMinRows;
     return host_pipeline(pl, X_host, N, ldx, P_out_host, ldp, [&](const float* x, int64_t n, float* p, cudaStream_t st, int) {
-        return launch_solve(pl, x, n, pl->F, max_evals, p, np, nullptr, st, proj_min);
+        return launch_solve(pl, x, n, pl->F, ipd, max_evals, p, np, nullptr, st, proj_min);
     });
+}
+}  // namespace
+
+extern "C" int nlml_tucker_fit_f32(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int iters,
+                                   float lr, float clip, float* P_out_dev, int64_t ldp, int kernel_hint,
+                                   void* stream) {
+    return fit_device(pl, X_dev, N, ldx, 0, iters, lr, clip, P_out_dev, ldp, kernel_hint, stream);
+}
+extern "C" int nlml_tucker_fit_landmarks_f32(nlml_tucker_plan* pl, const float* LM_dev, int64_t N, int64_t ldx, int iters,
+                                             float lr, float clip, float* P_out_dev, int64_t ldp, int kernel_hint,
+                                             void* stream) {
+    return fit_device(pl, LM_dev, N, ldx, 1, iters, lr, clip, P_out_dev, ldp, kernel_hint, stream);
+}
+
+extern "C" int nlml_tucker_fit_host_f32(nlml_tucker_plan* pl, const float* X_host, int64_t N, int64_t ldx,
+                                        int iters, float lr, float clip, float* P_out_host, int64_t ldp) {
+    return fit_host(pl, X_host, N, ldx, 0, iters, lr, clip, P_out_host, ldp);
+}
+extern "C" int nlml_tucker_fit_landmarks_host_f32(nlml_tucker_plan* pl, const float* LM_host, int64_t N, int64_t ldx,
+                                                  int iters, float lr, float clip, float* P_out_host, int64_t ldp) {
+    return fit_host(pl, LM_host, N, ldx, 1, iters, lr, clip, P_out_host, ldp);
+}
+
+extern "C" int nlml_tucker_solve_f32(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int max_evals,
+                                     float* P_out_dev, int64_t ldp, int32_t* evals_out_dev, void* stream) {
+    return solve_device(pl, X_dev, N, ldx, 0, max_evals, P_out_dev, ldp, evals_out_dev, stream);
+}
+extern "C" int nlml_tucker_solve_landmarks_f32(nlml_tucker_plan* pl, const float* LM_dev, int64_t N, int64_t ldx, int max_evals,
+                                               float* P_out_dev, int64_t ldp, int32_t* evals_out_dev, void* stream) {
+    return solve_device(pl, LM_dev, N, ldx, 1, max_evals, P_out_dev, ldp, evals_out_dev, stream);
+}
+
+extern "C" int nlml_tucker_solve_host_f32(nlml_tucker_plan* pl, const float* X_host, int64_t N, int64_t ldx,
+                                          int max_evals, float* P_out_host, int64_t ldp) {
+    return solve_host(pl, X_host, N, ldx, 0, max_evals, P_out_host, ldp);
+}
+extern "C" int nlml_tucker_solve_landmarks_host_f32(nlml_tucker_plan* pl, const float* LM_host, int64_t N, int64_t ldx,
+                                                    int max_evals, float* P_out_host, int64_t ldp) {
+    return solve_host(pl, LM_host, N, ldx, 1, max_evals, P_out_host, ldp);
 }
 
 #ifdef NLML_GEN_TIMING
@@ -2337,20 +2450,25 @@ static void pairwise_plan(int off, int n, std::vector<short>& loff, std::vector<
     prog.push_back(-1);
 }
 
-static int powell_launch(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, double* P_out_dev, int64_t ldp,
+static int powell_launch(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int ipd, double* P_out_dev, int64_t ldp,
                          double* fun_out_dev, int32_t* nfev_out_dev, void* stream, const double* pts, int npts, double* vals);
 
 extern "C" int nlml_tucker_powell_f64(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, double* P_out_dev,
                                       int64_t ldp, double* fun_out_dev, int32_t* nfev_out_dev, void* stream) {
     if (!pl || (N > 0 && (!X_dev || !P_out_dev))) return set_error(NLML_E_INVALID, "null pointer argument");
-    return powell_launch(pl, X_dev, N, ldx, P_out_dev, ldp, fun_out_dev, nfev_out_dev, stream, nullptr, 0, nullptr);
+    return powell_launch(pl, X_dev, N, ldx, 0, P_out_dev, ldp, fun_out_dev, nfev_out_dev, stream, nullptr, 0, nullptr);
+}
+extern "C" int nlml_tucker_powell_landmarks_f64(nlml_tucker_plan* pl, const float* LM_dev, int64_t N, int64_t ldx, double* P_out_dev,
+                                                int64_t ldp, double* fun_out_dev, int32_t* nfev_out_dev, void* stream) {
+    if (!pl || (N > 0 && (!LM_dev || !P_out_dev))) return set_error(NLML_E_INVALID, "null pointer argument");
+    return powell_launch(pl, LM_dev, N, ldx, 1, P_out_dev, ldp, fun_out_dev, nfev_out_dev, stream, nullptr, 0, nullptr);
 }
 /* test hook: q = W2 x of the tensor-core projection GEMM for N >= 4096 samples, CTA-blocked: Q_out_dev [ceil(N/128)][136][128] */
 extern "C" int nlml_debug_project_tc(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, float* Q_out_dev) {
     if (!pl || !X_dev || !Q_out_dev) return set_error(NLML_E_INVALID, "null pointer argument");
     DeviceGuard guard(pl->device);
     const float* q = nullptr;
-    if (int rc = project_tc(pl, X_dev, N, ldx, nullptr, &q)) return rc;
+    if (int rc = project_tc(pl, X_dev, N, ldx, 0, nullptr, &q)) return rc;
     if (!q) return set_error(NLML_E_UNSUPPORTED, "the tensor-core projection needs ranks (5,3,3,3), N >= 4096 and 16-byte aligned rows");
     NLML_CUDA(cudaEventRecord(pl->q_pre_done, nullptr));
     NLML_CUDA(cudaMemcpy(Q_out_dev, q, sizeof(float) * (size_t)ceil_div(N, 128) * 136 * 128, cudaMemcpyDeviceToDevice));
@@ -2359,20 +2477,21 @@ extern "C" int nlml_debug_project_tc(nlml_tucker_plan* pl, const float* X_dev, i
 /* test hook: TD_Tester.objective (float64, the reference's operation order) of ONE sample x at npts parameter points */
 extern "C" int nlml_debug_powell_objective(nlml_tucker_plan* pl, const float* x_dev, const double* pts_dev, int npts, double* vals_dev) {
     if (!pl || !x_dev || !pts_dev || !vals_dev || npts < 1) return set_error(NLML_E_INVALID, "null pointer argument");
-    return powell_launch(pl, x_dev, 1, pl->F, nullptr, 3 + pl->ri, nullptr, nullptr, nullptr, pts_dev, npts, vals_dev);
+    return powell_launch(pl, x_dev, 1, pl->F, 0, nullptr, 3 + pl->ri, nullptr, nullptr, nullptr, pts_dev, npts, vals_dev);
 }
-static int powell_launch(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, double* P_out_dev, int64_t ldp,
+static int powell_launch(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, int ipd, double* P_out_dev, int64_t ldp,
                          double* fun_out_dev, int32_t* nfev_out_dev, void* stream, const double* pts, int npts, double* vals) {
     if (N < 0 || ldx < pl->F || ldp < 3 + pl->ri)
         return set_error(NLML_E_INVALID, "bad sizes: N=%lld ldx=%lld (F=%d) ldp=%lld (need >= %d)", (long long)N, (long long)ldx, pl->F,
                          (long long)ldp, 3 + pl->ri);
+    if (int rc = check_landmark_plan(pl, ipd)) return rc;
     if (pl->F > kPowellThreads * kPowellMaxFeat || pl->F > 32000)
         return set_error(NLML_E_UNSUPPORTED, "the Powell fit serves F <= %d", kPowellThreads * kPowellMaxFeat);
     if (N == 0) return 0;
     DeviceGuard guard(pl->device);
     PowellArgs a{};
     a.X = X_dev; a.N = N; a.ldx = ldx; a.W2 = pl->W2; a.P = P_out_dev; a.ldp = ldp; a.fun = fun_out_dev; a.nfev = nfev_out_dev;
-    a.ri = pl->ri; a.ry = pl->ry; a.rp = pl->rp; a.rr = pl->rr; a.F = pl->F;
+    a.ri = pl->ri; a.ry = pl->ry; a.rp = pl->rp; a.rr = pl->rr; a.F = pl->F; a.ipd = ipd;
     std::vector<short> loff, llen;
     std::vector<signed char> prog;
     pairwise_plan(0, pl->F, loff, llen, prog);
@@ -2448,7 +2567,7 @@ extern "C" int nlml_core_times_features_f32(const float* core_host, const float*
     // the projection kernel computes rows(core) . rows(U_feat) in its CTA-blocked layout [R/128][F][128]
     const int vec_ok = (M % 4 == 0);
     tgen::tucker_project_kernel<<<dim3((unsigned)(Rp / 128), (unsigned)ceil_div(F, 64)), 256>>>((const float*)dc.p, R, M, (const float*)du.p, F, M, vec_ok,
-                                                                                               (float*)dq.p);
+                                                                                               (float*)dq.p, 0);
     NLML_CUDA(cudaGetLastError());
     std::vector<float> blocked((size_t)Rp * F);
     NLML_CUDA(cudaMemcpy(blocked.data(), dq.p, sizeof(float) * Rp * F, cudaMemcpyDeviceToHost));

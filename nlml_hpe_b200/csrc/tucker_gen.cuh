@@ -708,15 +708,22 @@ __global__ void __launch_bounds__(kThreads, 1) tucker_fit_gen_kernel(const __gri
 
 // q = W2 x for a batch, written as the CTA-blocked slabs the generic kernel reads: Q[(s / 128) * R + r][s % 128].
 // Plain FP32 tiled GEMM (128 samples x 64 rows of W2 per block, 16 features per step): one pass, ~1 % of a T = 3000 fit.
+// ipd: the X rows are raw landmarks; the block derives its 128 rows' (ref, ipd) once and applies the IPD normalisation
+// (common.cuh) to each staged X tile.
 __global__ void __launch_bounds__(256) tucker_project_kernel(const float* __restrict__ X, long long N, long long ldx,
                                                             const float* __restrict__ W2, int R, int F, int vec_ok,
-                                                            float* __restrict__ Q) {
+                                                            float* __restrict__ Q, int ipd) {
     constexpr int BM = 128, BR = 64, BK = 16;
     __shared__ __align__(16) float Xs[BK][BM + 4];
     __shared__ __align__(16) float Ws[BK][BR + 4];
+    extern __shared__ IpdRow ipd_s[];   // [BM], launched with sizeof(IpdRow) * BM bytes of dynamic shared memory when ipd
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;   // tx: 16 sample groups (sample = tx + 16 i), ty: 16 row groups of 4
     const long long m0 = (long long)blockIdx.x * BM;
     const int r0 = blockIdx.y * BR;
+    if (ipd) {
+        if (tid < BM && m0 + tid < N) ipd_s[tid] = ipd_row(X + (m0 + tid) * ldx);
+        __syncthreads();
+    }
     float acc[8][4];
 #pragma unroll
     for (int i = 0; i < 8; ++i)
@@ -756,6 +763,10 @@ __global__ void __launch_bounds__(256) tucker_project_kernel(const float* __rest
             Ws[4 * c4 + 0][r] = v.x; Ws[4 * c4 + 1][r] = v.y; Ws[4 * c4 + 2][r] = v.z; Ws[4 * c4 + 3][r] = v.w;
         }
         __syncthreads();
+        if (ipd) {
+            ipd_tile(&Xs[0][0], BM + 4, BK, BM, ipd_s, N - m0, f0, F, tid, 256);
+            __syncthreads();
+        }
 #pragma unroll
         for (int k = 0; k < BK; ++k) {
             float xv[8];

@@ -18,6 +18,13 @@ KERNEL_HINTS = {"auto": 0, "thread_per_sample": 1, "cta_per_sample": 2, "warp_pe
                 "thread_per_sample_tmem": 4, "tensor_core": 5, "tensor_core_generic": 6}
 
 
+def _flatten_landmarks(X, landmarks):
+    """Raw MediaPipe landmarks [N,468,3] -> [N,1404] (x,y,z of landmark i at columns 3i..3i+2); anything else as given."""
+    if landmarks and X.ndim == 3 and X.shape[2] == 3:
+        return X.reshape(X.shape[0], X.shape[1] * 3)
+    return X
+
+
 def _device_index(device):
     if device is None:
         return torch.cuda.current_device() if torch.cuda.is_available() else 0
@@ -34,6 +41,12 @@ class TuckerFitter:
     params_*: [R_a, 4] rows (a,b,c,d) of optimized_{yaw,pitch,roll} (TD_Inference.py:43-45);
     ranks are taken from W, and the first R_a rows of each params array are used
     (the reference hard-slices [0:3,:], TD_Inference.py:56-57).
+
+    Every fit / solve / powell entry point takes landmarks=True for RAW MediaPipe landmarks ([N,468,3] or [N,>=F],
+    x,y,z of landmark i at columns 3i..3i+2): the IPD normalisation of
+    FeatureExtractor.Read_Landmarks_and_Normalizing_using_IPD (helpers/FeatureExtractor.py:30-66) then runs inside the
+    kernels' reads of X, in float64 as the reference, and the result equals the call on the normalised features bit
+    for bit.  Needs F >= 792 (landmark 263).
     """
 
     def __init__(self, W, params_y, params_p, params_r, device=None):
@@ -74,14 +87,16 @@ class TuckerFitter:
     def launches(self):
         return int(self._lib.nlml_tucker_launch_count(self._h))
 
-    def fit(self, X, iters=3000, lr=1e-3, clip=1.0, kernel="auto", out=None):
-        """X: CUDA float32 tensor [N, >=F] (row stride arbitrary, unit column stride).
+    def fit(self, X, iters=3000, lr=1e-3, clip=1.0, kernel="auto", out=None, landmarks=False):
+        """X: CUDA float32 tensor [N, >=F] (row stride arbitrary, unit column stride); with landmarks=True raw
+        landmarks [N,468,3] or [N,>=F] (see the class docstring).
 
         Returns a CUDA tensor [N, 3+R_id]: (yaw, pitch, roll) in radians + identity coefficients,
         the vector optimize_with_sgd returns (TD_Tester.py:159).  Asynchronous on the current stream.
         """
         if not (isinstance(X, torch.Tensor) and X.is_cuda):
             raise TypeError("fit() takes a CUDA tensor; use fit_host() for numpy / CPU tensors")
+        X = _flatten_landmarks(X, landmarks)
         if X.dtype != torch.float32 or X.dim() != 2 or X.shape[1] < self.F:
             raise ValueError(f"X must be float32 [N, >={self.F}], got {X.dtype} {tuple(X.shape)}")
         if X.device.index != self.device_index:
@@ -93,18 +108,19 @@ class TuckerFitter:
             out = torch.empty((n, self.n_params), dtype=torch.float32, device=X.device)
         stream = torch.cuda.current_stream(X.device).cuda_stream
         ldx = X.stride(0) if n > 1 else max(X.shape[1], self.F)
-        _lib.check(self._lib.nlml_tucker_fit_f32(self._h, X.data_ptr(), n, ldx, int(iters), float(lr), float(clip),
-                                                 out.data_ptr(), out.stride(0) if n > 1 else self.n_params,
-                                                 KERNEL_HINTS[kernel], stream))
+        call = self._lib.nlml_tucker_fit_landmarks_f32 if landmarks else self._lib.nlml_tucker_fit_f32
+        _lib.check(call(self._h, X.data_ptr(), n, ldx, int(iters), float(lr), float(clip),
+                        out.data_ptr(), out.stride(0) if n > 1 else self.n_params, KERNEL_HINTS[kernel], stream))
         return out
 
-    def solve(self, X, max_evals=0, return_evals=False, out=None):
+    def solve(self, X, max_evals=0, return_evals=False, out=None, landmarks=False):
         """Converged fit (what TD_Tester.Test computes with scipy Powell, TD_Tester.py:191-199): damped Newton
-        from p = 0 to the local minimum, one thread per sample.  X as in fit().  Returns [N, 3+R_id]
+        from p = 0 to the local minimum, one thread per sample.  X (and landmarks) as in fit().  Returns [N, 3+R_id]
         (radians + identity coefficients) and, with return_evals, the int32 [N] evaluations used.
         Ranks (5,3,3,3) only.  Asynchronous on the current stream."""
         if not (isinstance(X, torch.Tensor) and X.is_cuda):
             raise TypeError("solve() takes a CUDA tensor; use solve_host() for numpy / CPU tensors")
+        X = _flatten_landmarks(X, landmarks)
         if X.dtype != torch.float32 or X.dim() != 2 or X.shape[1] < self.F:
             raise ValueError(f"X must be float32 [N, >={self.F}], got {X.dtype} {tuple(X.shape)}")
         if X.device.index != self.device_index:
@@ -117,19 +133,23 @@ class TuckerFitter:
         evals = torch.zeros((n,), dtype=torch.int32, device=X.device) if return_evals else None
         stream = torch.cuda.current_stream(X.device).cuda_stream
         ldx = X.stride(0) if n > 1 else max(X.shape[1], self.F)
-        _lib.check(self._lib.nlml_tucker_solve_f32(self._h, X.data_ptr(), n, ldx, int(max_evals), out.data_ptr(),
-                                                   out.stride(0) if n > 1 else self.n_params,
-                                                   evals.data_ptr() if return_evals and n > 0 else None, stream))
+        call = self._lib.nlml_tucker_solve_landmarks_f32 if landmarks else self._lib.nlml_tucker_solve_f32
+        _lib.check(call(self._h, X.data_ptr(), n, ldx, int(max_evals), out.data_ptr(),
+                        out.stride(0) if n > 1 else self.n_params,
+                        evals.data_ptr() if return_evals and n > 0 else None, stream))
         return (out, evals) if return_evals else out
 
-    def powell(self, X, return_info=False):
+    def powell(self, X, return_info=False, landmarks=False):
         """The reference's shipped default fit, bit for bit: scipy Powell from p = 0 over TD_Tester.objective
         (TD_Tester.py:31-58, :191-194; algorithm restated from scipy 1.18.1 in csrc/powell_math.h, objective evaluated in
         the reference's own operation order).  X: CUDA float32 [N, >=F].  Returns a CUDA float64 tensor [N, 3+R_id] =
         result.x (radians + identity coefficients) and, with return_info, (result.fun float64 [N], result.nfev int32 [N]).
-        One CTA per sample, float64: ~10^4 poses/s -- use solve() / fit() for throughput.  Asynchronous."""
+        One CTA per sample, float64: ~10^4 poses/s -- use solve() / fit() for throughput.  Asynchronous.
+        With landmarks=True (see the class docstring) it equals the reference's
+        FE.get_feature_vector(..., normalize=True) -> Test() chain."""
         if not (isinstance(X, torch.Tensor) and X.is_cuda):
             raise TypeError("powell() takes a CUDA tensor")
+        X = _flatten_landmarks(X, landmarks)
         if X.dtype != torch.float32 or X.dim() != 2 or X.shape[1] < self.F:
             raise ValueError(f"X must be float32 [N, >={self.F}], got {X.dtype} {tuple(X.shape)}")
         if X.device.index != self.device_index:
@@ -142,39 +162,41 @@ class TuckerFitter:
         nfev = torch.empty((n,), dtype=torch.int32, device=X.device) if return_info else None
         stream = torch.cuda.current_stream(X.device).cuda_stream
         ldx = X.stride(0) if n > 1 else max(X.shape[1], self.F)
-        _lib.check(self._lib.nlml_tucker_powell_f64(self._h, X.data_ptr(), n, ldx, out.data_ptr(), self.n_params,
-                                                    fun.data_ptr() if return_info and n > 0 else None,
-                                                    nfev.data_ptr() if return_info and n > 0 else None, stream))
+        call = self._lib.nlml_tucker_powell_landmarks_f64 if landmarks else self._lib.nlml_tucker_powell_f64
+        _lib.check(call(self._h, X.data_ptr(), n, ldx, out.data_ptr(), self.n_params,
+                        fun.data_ptr() if return_info and n > 0 else None,
+                        nfev.data_ptr() if return_info and n > 0 else None, stream))
         return (out, fun, nfev) if return_info else out
 
-    def solve_host(self, X, max_evals=0, out=None):
-        """solve() for numpy / CPU float32 [N, F] in host memory; pipelined like fit_host()."""
+    def solve_host(self, X, max_evals=0, out=None, landmarks=False):
+        """solve() for numpy / CPU float32 [N, F] in host memory (or raw landmarks with landmarks=True); pipelined like
+        fit_host()."""
         if isinstance(X, torch.Tensor):
             X = X.detach().numpy()
-        X = np.asarray(X)
+        X = _flatten_landmarks(np.asarray(X), landmarks)
         if X.dtype != np.float32 or X.ndim != 2 or X.shape[1] < self.F or (X.size and X.strides[1] != 4):
             raise ValueError(f"X must be float32 [N, >={self.F}] with unit column stride")
         n = X.shape[0]
         if out is None:
             out = np.empty((n, self.n_params), dtype=np.float32)
         ldx = X.strides[0] // 4 if n > 1 else X.shape[1]
-        _lib.check(self._lib.nlml_tucker_solve_host_f32(self._h, X.ctypes.data, n, ldx, int(max_evals),
-                                                        out.ctypes.data, self.n_params))
+        call = self._lib.nlml_tucker_solve_landmarks_host_f32 if landmarks else self._lib.nlml_tucker_solve_host_f32
+        _lib.check(call(self._h, X.ctypes.data, n, ldx, int(max_evals), out.ctypes.data, self.n_params))
         return out
 
-    def fit_host(self, X, iters=3000, lr=1e-3, clip=1.0, out=None):
+    def fit_host(self, X, iters=3000, lr=1e-3, clip=1.0, out=None, landmarks=False):
         """X: numpy / CPU tensor float32 [N, F] in host memory (pinned memory makes the copies
-        asynchronous).  Host->device copy, fit and device->host copy are pipelined inside the
-        library.  Returns numpy float32 [N, 3+R_id]."""
+        asynchronous); with landmarks=True raw landmarks [N,468,3] or [N,>=F].  Host->device copy, fit and
+        device->host copy are pipelined inside the library.  Returns numpy float32 [N, 3+R_id]."""
         if isinstance(X, torch.Tensor):
             X = X.detach().numpy()
-        X = np.asarray(X)
+        X = _flatten_landmarks(np.asarray(X), landmarks)
         if X.dtype != np.float32 or X.ndim != 2 or X.shape[1] < self.F or (X.size and X.strides[1] != 4):
             raise ValueError(f"X must be float32 [N, >={self.F}] with unit column stride")
         n = X.shape[0]
         if out is None:
             out = np.empty((n, self.n_params), dtype=np.float32)
         ldx = X.strides[0] // 4 if n > 1 else X.shape[1]
-        _lib.check(self._lib.nlml_tucker_fit_host_f32(self._h, X.ctypes.data, n, ldx, int(iters), float(lr),
-                                                      float(clip), out.ctypes.data, self.n_params))
+        call = self._lib.nlml_tucker_fit_landmarks_host_f32 if landmarks else self._lib.nlml_tucker_fit_host_f32
+        _lib.check(call(self._h, X.ctypes.data, n, ldx, int(iters), float(lr), float(clip), out.ctypes.data, self.n_params))
         return out
