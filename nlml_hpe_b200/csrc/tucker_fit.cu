@@ -866,13 +866,45 @@ __global__ void build_tc_operands_kernel(const float* __restrict__ S, float s_sc
     }
 }
 
+// Packed FP32 (f32x2) forms of the tensor-core kernel's scalar products: each lane does the scalar code's IEEE operation,
+// so the results are bit for bit those of the scalar loops they replace.
+// y[i] = x[i] * k
+template <int N>
+__device__ __forceinline__ void scale_packed(const float* x, float k, float* y) {
+#pragma unroll
+    for (int i = 0; i + 1 < N; i += 2) {
+        const float2 t = __fmul2_rn(make_float2(x[i], x[i + 1]), make_float2(k, k));
+        y[i] = t.x;
+        y[i + 1] = t.y;
+    }
+    if (N % 2) y[N - 1] = x[N - 1] * k;
+}
+// sym_products with one factor pre-scaled: vv[(i,j)] = vs[i] * v[j] for i <= j, paired along even j within a row
+template <int R>
+__device__ __forceinline__ void sym_products_packed(const float* vs, const float* v, float* vv) {
+#pragma unroll
+    for (int i = 0; i < R; ++i)
+#pragma unroll
+        for (int j = i; j < R; ++j) {
+            if (j % 2 == 0 && j + 1 < R) {
+                const float2 t = __fmul2_rn(make_float2(vs[i], vs[i]), make_float2(v[j], v[j + 1]));
+                vv[pair_index(i, j, R)] = t.x;
+                vv[pair_index(i, j + 1, R)] = t.y;
+            } else if (j % 2 == 0 || j == i) {
+                vv[pair_index(i, j, R)] = vs[i] * v[j];
+            }
+        }
+}
+
 // All of T contracted over b first: s[c,d] = sum_b T[b,c,d] * YYk[b] (216 FMAs; YYk carries the inverse operand scales).
 // GR[d] = sum_c PP_c s[c,d] and GP[c] = sum_d RR_d s[c,d] follow from it (72 FMAs); GY comes from the V accumulator
 // (GY[b] = sum_A UU_A V[A,b], on the identity thread).  The earlier form (tr[b,c] = sum_d T RR_d for GY and GP, plus
 // GR on its own) took 504 FMAs on the angle thread.
-__device__ __forceinline__ void tc_reduce_t_b(uint32_t taddr, const float (&YYk)[6], float (&s)[36]) {
+// The FMAs run as 108 packed pairs s[c, d..d+1] (FFMA2, YYk[b] broadcast): column bcd = 36b + 6c + d, so an even column
+// starts a pair of one (b, c), and it sits in an aligned register pair of the load.  Each lane is the scalar fmaf chain.
+__device__ __forceinline__ void tc_reduce_t_b(uint32_t taddr, const float (&YYk)[6], float2 (&s)[18]) {
 #pragma unroll
-    for (int i = 0; i < 36; ++i) s[i] = 0.f;
+    for (int i = 0; i < 18; ++i) s[i] = make_float2(0.f, 0.f);
     constexpr int NL = 7;   // 224 columns, 216 used
     uint32_t buf[2][32];
     tmem_load32_async(taddr, buf[0]);
@@ -881,9 +913,13 @@ __device__ __forceinline__ void tc_reduce_t_b(uint32_t taddr, const float (&YYk)
         tmem_load_wait();
         if (ci + 1 < NL) tmem_load32_async(taddr + 32 * (ci + 1), buf[(ci + 1) & 1]);
 #pragma unroll
-        for (int x = 0; x < 32; ++x) {
+        for (int x = 0; x < 32; x += 2) {
             const int bcd = 32 * ci + x;
-            if (bcd < 216) s[bcd % 36] = fmaf(__uint_as_float(buf[ci & 1][x]), YYk[bcd / 36], s[bcd % 36]);
+            if (bcd < 216) {
+                const float2 t = make_float2(__uint_as_float(buf[ci & 1][x]), __uint_as_float(buf[ci & 1][x + 1]));
+                const float y = YYk[bcd / 36];
+                s[(bcd % 36) / 2] = __ffma2_rn(t, make_float2(y, y), s[(bcd % 36) / 2]);
+            }
         }
     }
 }
@@ -1055,20 +1091,16 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
             {
                 const float su = __int_as_float((eu + 127) << 23);
                 float us[5];   // the scale rides on one factor of every product (exact: a power of two)
-#pragma unroll
-                for (int i = 0; i < 5; ++i) us[i] = u[i] * su;
-#pragma unroll
-                for (int i = 0; i < 5; ++i)
-#pragma unroll
-                    for (int j = i; j < 5; ++j) UU[pair_index(i, j, 5)] = us[i] * u[j];
+                scale_packed<5>(u, su, us);
+                sym_products_packed<5>(us, u, UU);
                 UU[15] = 0.f;
             }
 #pragma unroll
             for (int k2 = 0; k2 < 8; ++k2) {   // packed pairs: element 2c in the low half of column c
-                const float v0 = UU[2 * k2], v1 = UU[2 * k2 + 1];
-                const __half2 h = __floats2half2_rn(v0, v1);
+                const float2 v = make_float2(UU[2 * k2], UU[2 * k2 + 1]);
+                const __half2 h = __float22half2_rn(v);
                 const float2 hf = __half22float2(h);
-                const __half2 l = __floats2half2_rn(v0 - hf.x, v1 - hf.y);
+                const __half2 l = __float22half2_rn(__fadd2_rn(v, make_float2(-hf.x, -hf.y)));
                 hl[k2] = __uint_as_float(*reinterpret_cast<const uint32_t*>(&h));
                 hl[8 + k2] = __uint_as_float(*reinterpret_cast<const uint32_t*>(&l));
             }
@@ -1103,20 +1135,20 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
             float PPs[6];   // the operand's power-of-two scale rides on PP
             {
                 const float kPrScale = __int_as_float((127 + a.pr_exp) << 23);
-#pragma unroll
-                for (int i = 0; i < 6; ++i) PPs[i] = PP[i] * kPrScale;
+                scale_packed<6>(PP, kPrScale, PPs);
             }
 #pragma unroll
             for (int k8 = 0; k8 < C::KV / 8; ++k8) {   // one 16-byte chunk = 8 halves of this row per plane
                 uint32_t wh[4], wl[4];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
-                    const int k0 = 8 * k8 + 2 * e, k1 = k0 + 1;
-                    const float v0 = k0 < 36 ? PPs[k0 / 6] * RRv[k0 % 6] : 0.f;
-                    const float v1 = k1 < 36 ? PPs[k1 / 6] * RRv[k1 % 6] : 0.f;
-                    const __half2 h = __floats2half2_rn(v0, v1);
+                    const int k0 = 8 * k8 + 2 * e;   // k = 6c + D: an even k starts a pair (D, D+1) of one c
+                    const float2 v = k0 < 36 ? __fmul2_rn(make_float2(PPs[k0 / 6], PPs[k0 / 6]),
+                                                          make_float2(RRv[k0 % 6], RRv[k0 % 6 + 1]))
+                                             : make_float2(0.f, 0.f);
+                    const __half2 h = __float22half2_rn(v);
                     const float2 hf = __half22float2(h);
-                    const __half2 l = __floats2half2_rn(v0 - hf.x, v1 - hf.y);
+                    const __half2 l = __float22half2_rn(__fadd2_rn(v, make_float2(-hf.x, -hf.y)));
                     wh[e] = *reinterpret_cast<const uint32_t*>(&h);
                     wl[e] = *reinterpret_cast<const uint32_t*>(&l);
                 }
@@ -1154,20 +1186,16 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
             float GU[15], GYv[6], YYk[6], UUk[15];
             {
                 const float kv = __int_as_float((127 - a.s_exp - a.pr_exp) << 23);   // 2^-(s_exp + pr_exp): the V accumulator's scale off
-#pragma unroll
-                for (int i = 0; i < 6; ++i) YYk[i] = YY[i] * kv;
+                scale_packed<6>(YY, kv, YYk);
                 float uk[5];   // the scale rides on one factor of every product
-#pragma unroll
-                for (int i = 0; i < 5; ++i) uk[i] = u[i] * kv;
-#pragma unroll
-                for (int i = 0; i < 5; ++i)
-#pragma unroll
-                    for (int j = i; j < 5; ++j) UUk[pair_index(i, j, 5)] = uk[i] * u[j];
+                scale_packed<5>(u, kv, uk);
+                sym_products_packed<5>(uk, u, UUk);
             }
+            float2 GY2[3];   // GY[b..b+1] as packed pairs (UUk[A] broadcast); GU[A] stays one scalar chain per A
 #pragma unroll
             for (int i = 0; i < 15; ++i) GU[i] = 0.f;
 #pragma unroll
-            for (int i = 0; i < 6; ++i) GYv[i] = 0.f;
+            for (int i = 0; i < 3; ++i) GY2[i] = make_float2(0.f, 0.f);
             if (NLML_DBG_MMA) ttc::mbar_wait(bar + 1, phase);   // V GEMM
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             NLML_TSTAMP(3);   // wait for the GEMM
@@ -1179,15 +1207,21 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
                     tmem_load_wait();
                     if (ci + 1 < C::NV / 32) tmem_load32_async(lane_addr + C::COL_V + 32 * (ci + 1), vb[(ci + 1) & 1]);
 #pragma unroll
-                    for (int x = 0; x < 32; ++x) {
+                    for (int x = 0; x < 32; x += 2) {   // column n = 6A + b: an even column starts a pair (b, b+1) of one A
                         const int n = 32 * ci + x;
                         if (n < 90) {
-                            const float v = __uint_as_float(vb[ci & 1][x]);
-                            GU[n / 6] = fmaf(v, YYk[n % 6], GU[n / 6]);
-                            GYv[n % 6] = fmaf(v, UUk[n / 6], GYv[n % 6]);
+                            const float2 v = make_float2(__uint_as_float(vb[ci & 1][x]), __uint_as_float(vb[ci & 1][x + 1]));
+                            GU[n / 6] = fmaf(v.x, YYk[n % 6], GU[n / 6]);
+                            GU[n / 6] = fmaf(v.y, YYk[n % 6 + 1], GU[n / 6]);
+                            GY2[(n % 6) / 2] = __ffma2_rn(v, make_float2(UUk[n / 6], UUk[n / 6]), GY2[(n % 6) / 2]);
                         }
                     }
                 }
+            }
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                GYv[2 * i] = GY2[i].x;
+                GYv[2 * i + 1] = GY2[i].y;
             }
             float du[5], dy[3];
             sym_backprop<5>(GU, u, du);
@@ -1197,26 +1231,35 @@ __global__ void __launch_bounds__(256, 1) tucker_fit_tc_kernel(const __grid_cons
             gx[8 * 128 + row] = fmaf(dy[2], dcy[2], fmaf(dy[1], dcy[1], dy[0] * dcy[0]));   // the angle thread adds -ey.dcy
         } else {
             // all of T -> s[c,d] -> GR, GP -> d/d(pitch, roll); d/d(yaw): the linear part here, the quadratic part on the identity thread
-            float GR[6], GP[6], sc[36], YYk[6];
+            float GR[6], GP[6], YYk[6];
+            float2 sc[18];
             {
                 const float kt = __int_as_float((127 - a.s_exp - uu_exp) << 23);   // 2^-(s_exp + uu_exp): the T accumulator's scale off
-#pragma unroll
-                for (int i = 0; i < 6; ++i) YYk[i] = YY[i] * kt;
+                scale_packed<6>(YY, kt, YYk);
             }
             if (NLML_DBG_MMA) ttc::mbar_wait(bar, phase);       // T GEMM (launched first, long done)
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             NLML_TSTAMP(3);
+            float2 GR2[3];   // GR[d..d+1] as packed pairs (PP_c broadcast); GP[c] stays one scalar chain per c
 #pragma unroll
-            for (int i = 0; i < 6; ++i) GR[i] = GP[i] = 0.f;
+            for (int i = 0; i < 3; ++i) GR2[i] = make_float2(0.f, 0.f);
+#pragma unroll
+            for (int i = 0; i < 6; ++i) GP[i] = 0.f;
             if (NLML_DBG_READ) {
                 tc_reduce_t_b(lane_addr + C::COL_T, YYk, sc);
 #pragma unroll
                 for (int c = 0; c < 6; ++c)
 #pragma unroll
-                    for (int d = 0; d < 6; ++d) {
-                        GR[d] = fmaf(PP[c], sc[c * 6 + d], GR[d]);
-                        GP[c] = fmaf(RRv[d], sc[c * 6 + d], GP[c]);
+                    for (int d2 = 0; d2 < 3; ++d2) {
+                        GR2[d2] = __ffma2_rn(make_float2(PP[c], PP[c]), sc[c * 3 + d2], GR2[d2]);
+                        GP[c] = fmaf(RRv[2 * d2], sc[c * 3 + d2].x, GP[c]);
+                        GP[c] = fmaf(RRv[2 * d2 + 1], sc[c * 3 + d2].y, GP[c]);
                     }
+            }
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                GR[2 * i] = GR2[i].x;
+                GR[2 * i + 1] = GR2[i].y;
             }
             float dp[3], dr[3];
             sym_backprop<3>(GP, cp, dp);
