@@ -121,6 +121,13 @@ int nlml_tucker_powell_landmarks_f64(nlml_tucker_plan* plan, const float* LM_dev
  * (q[r] of sample s at ((s / 128) * 136 + r) * 128 + s % 128).  Synchronous. */
 int nlml_debug_project_tc(nlml_tucker_plan* plan, const float* X_dev, int64_t N, int64_t ldx, float* Q_out_dev);
 
+/* Test hook: the configuration the run-time-rank tensor-core kernel (tucker_fit_gen_kernel) gets for ranks
+ * (r_id, r_y, r_p, r_r), as plan creation chooses it.  No CUDA call: works without a device.  out[0..22] =
+ * rrmax, nA, KA, NA16, nBC, nDp, BCP, NB, nblocks, resident, tslots, gslots, ypr_tmem, tbufs, gbufs, ybufs,
+ * col_g, col_a, col_t, col_y, smem_bytes, tt_bytes, gt_bytes (n_out >= 23).  NLML_E_UNSUPPORTED, with the
+ * reason in nlml_last_error(), when the kernel cannot serve the ranks. */
+int nlml_debug_gen_config(int r_id, int r_y, int r_p, int r_r, int32_t* out, int n_out);
+
 /* Test hook: TD_Tester.objective of ONE sample x_dev [F] at npts parameter points pts_dev [npts][3 + r_id] (float64),
  * evaluated by the Powell kernel's cooperative objective -> vals_dev [npts]. */
 int nlml_debug_powell_objective(nlml_tucker_plan* plan, const float* x_dev, const double* pts_dev, int npts, double* vals_dev);

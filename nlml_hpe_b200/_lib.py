@@ -19,7 +19,7 @@ EXPORTS = [
     "nlml_tucker_fit_host_f32", "nlml_tucker_solve_f32", "nlml_tucker_solve_host_f32", "nlml_tucker_launch_count",
     "nlml_tucker_fit_landmarks_f32", "nlml_tucker_fit_landmarks_host_f32", "nlml_tucker_solve_landmarks_f32",
     "nlml_tucker_solve_landmarks_host_f32", "nlml_tucker_powell_landmarks_f64",
-    "nlml_tucker_powell_f64", "nlml_debug_powell_objective", "nlml_debug_project_tc", "nlml_cosine_fit_f64", "nlml_core_times_features_f32",
+    "nlml_tucker_powell_f64", "nlml_debug_powell_objective", "nlml_debug_project_tc", "nlml_debug_gen_config", "nlml_cosine_fit_f64", "nlml_core_times_features_f32",
     "nlml_mlp_plan_create", "nlml_mlp_plan_destroy", "nlml_mlp_forward_f32",
     "nlml_mlp_forward_host_f32", "nlml_mlp_forward_landmarks_f32", "nlml_mlp_forward_landmarks_host_f32", "nlml_pose_postprocess_f64", "nlml_mlp_latent_f32", "nlml_mlp_launch_count", "nlml_mlp_set_path",
     "nlml_measure_fp32_tflops", "nlml_measure_fp32_tflops_3reg", "nlml_measure_tf32_tflops", "nlml_debug_tf32_gemm", "nlml_debug_tf32_gemm_mode",
@@ -60,6 +60,7 @@ def load():
     lib.nlml_tucker_powell_landmarks_f64.argtypes = lib.nlml_tucker_powell_f64.argtypes
     lib.nlml_debug_powell_objective.argtypes = [vp, vp, vp, i32, vp]
     lib.nlml_debug_project_tc.argtypes = [vp, vp, i64, i64, vp]
+    lib.nlml_debug_gen_config.argtypes = [i32, i32, i32, i32, vp, i32]
     lib.nlml_cosine_fit_f64.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, i32]
     lib.nlml_core_times_features_f32.argtypes = [vp, vp, i64, i32, i32, vp, i32]
     lib.nlml_tucker_launch_count.argtypes = [vp]

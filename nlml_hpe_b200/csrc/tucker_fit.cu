@@ -1843,8 +1843,8 @@ size_t wps_smem_bytes(int F) { return sizeof(float) * kWpsWarps * ((F + 3) / 4 *
 
 // ---- run-time-rank tensor-core kernel: per-plan configuration (TMEM columns, shared-memory ring, block size) ----
 constexpr int kGenSmemMax = 232448;   // 227 KB of dynamic shared memory per CTA
+// ranks: roll <= 8, others <= tgen::kMaxRank (checked by gen_config_for)
 bool choose_gen_config(int ri, int ry, int rp, int rr, tgen::GenCfg& best) {
-    if (rr > 8 || ri > tgen::kMaxRank || ry > tgen::kMaxRank || rp > tgen::kMaxRank) return false;
     tgen::GenCfg b{};
     b.ri = ri; b.ry = ry; b.rp = rp; b.rr = rr; b.R = ri * ry * rp * rr;
     b.rrmax = rr <= 5 ? 5 : 8;
@@ -1855,7 +1855,10 @@ bool choose_gen_config(int ri, int ry, int rp, int rr, tgen::GenCfg& best) {
     b.t_p = 0; b.t_gx = b.NP; b.t_gl = 2 * b.NP; b.t_cy = 3 * b.NP; b.t_dcy = b.t_cy + ry; b.t_cp = b.t_dcy + ry;
     b.t_dcp = b.t_cp + rp; b.t_rows = b.t_dcp + rp;
     const int tab_bytes = b.t_rows * tgen::kSamples * 4, bar_bytes = 1024;
-    double best_score = -1.0;
+    // the highest-scoring feasible candidate, whatever its sign: roll rank 1 fills 1 of every 16 columns, so all of its
+    // candidates score below zero (ties keep the first candidate)
+    double best_score = -HUGE_VAL;
+    bool found = false;
 #ifdef NLML_GEN_TUNE
     // development build only (-DNLML_GEN_TUNE): pin parts of the configuration from the environment for sweeps
     auto pin = [](const char* name) { const char* e = std::getenv(name); return e ? std::atoi(e) : 0; };
@@ -1891,7 +1894,8 @@ bool choose_gen_config(int ri, int ry, int rp, int rr, tgen::GenCfg& best) {
                     // (16,8,8,8): NB = 80 with two ring slots 3226 poses/s, NB = 48 with three 2370)
                     const double score = (resident ? 40.0 : 10.0 * std::min(slots, 3)) + 6.0 * ybufs + 4.0 * tbufs + 3.0 * gbufs + 30.0 * ytm +
                                          (resident ? 0.25 : 0.6) * std::min(NB, 128) - 20.0 * waste;
-                    if (score <= best_score) continue;
+                    if (found && score <= best_score) continue;
+                    found = true;
                     best_score = score;
                     best = b;
                     best.BCP = BCP; best.NB = NB; best.nblocks = nblocks;
@@ -1908,7 +1912,31 @@ bool choose_gen_config(int ri, int ry, int rp, int rr, tgen::GenCfg& best) {
                 }
             }
     }
-    return best_score >= 0.0;
+    return found;
+}
+
+// Configuration of the run-time-rank tensor-core kernel for a rank set, or why it has none (nullptr on success).  Plan
+// creation and nlml_debug_gen_config both decide through this function.
+constexpr double kGenMaxTileBytes = 3.0e9;   // tile images of S kept on the device
+const char* gen_config_for(int ri, int ry, int rp, int rr, tgen::GenCfg& cfg) {
+    static thread_local char why[160];
+    if (rr > 8 || ri > tgen::kMaxRank || ry > tgen::kMaxRank || rp > tgen::kMaxRank) {
+        std::snprintf(why, sizeof(why), "the run-time-rank tensor-core kernel serves roll ranks <= 8 and other ranks <= %d "
+                      "(ranks %d,%d,%d,%d)", tgen::kMaxRank, ri, ry, rp, rr);
+        return why;
+    }
+    if (!choose_gen_config(ri, ry, rp, rr, cfg)) {
+        std::snprintf(why, sizeof(why), "no block size of the run-time-rank tensor-core kernel fits tensor memory and "
+                      "shared memory for ranks %d,%d,%d,%d", ri, ry, rp, rr);
+        return why;
+    }
+    const double tile_bytes = (double)cfg.nblocks * ((double)cfg.tt_bytes + cfg.gt_bytes);
+    if (tile_bytes > kGenMaxTileBytes) {
+        std::snprintf(why, sizeof(why), "the run-time-rank tensor-core kernel's tile images of ranks %d,%d,%d,%d would "
+                      "take %.2f GB (limit %.1f GB)", ri, ry, rp, rr, tile_bytes * 1e-9, kGenMaxTileBytes * 1e-9);
+        return why;
+    }
+    return nullptr;
 }
 
 template <int RRMAX, int NA16MAX>
@@ -1984,8 +2012,10 @@ int launch_fit(nlml_tucker_plan* pl, const float* X, int64_t N, int64_t ldx, int
                float* P, int64_t ldp, int hint, cudaStream_t st, int ws_slot = 2, int64_t proj_min_rows = kProjMinRows) {
     if (N == 0) return 0;
     // run-time-rank tensor-core kernel: asked for, or the default for every rank set without compiled kernels
-    if (hint == 6 && !pl->gen_ok)
-        return set_error(NLML_E_UNSUPPORTED, "the run-time-rank tensor-core kernel serves roll ranks <= 8 and other ranks <= %d", tgen::kMaxRank);
+    if (hint == 6 && !pl->gen_ok) {
+        tgen::GenCfg unused{};
+        return set_error(NLML_E_UNSUPPORTED, "%s", gen_config_for(pl->ri, pl->ry, pl->rp, pl->rr, unused));
+    }
     if (hint == 2 && !pl->cta_ok)
         return set_error(NLML_E_UNSUPPORTED, "core too large for the CTA-per-sample kernel's shared-memory working set");
     if (hint == 6 || (hint == 0 && !pl->fast && pl->gen_ok && (N >= 32 || !pl->cta_ok)))
@@ -2211,15 +2241,11 @@ extern "C" int nlml_tucker_plan_create(const float* W_host, int r_id, int r_y, i
     pl->NAP = (pl->nA + 3) / 4 * 4;
     pl->nBCD = tri(r_y) * tri(r_p) * tri(r_r);
     pl->nBCDp = (pl->nBCD + 31) / 32 * 32;
-    pl->gen_ok = choose_gen_config(r_id, r_y, r_p, r_r, pl->gen);
-    if (pl->gen_ok) {
-        const double tile_bytes = (double)pl->gen.nblocks * ((double)pl->gen.tt_bytes + pl->gen.gt_bytes);
-        if (tile_bytes > 3.0e9) pl->gen_ok = false;
-    }
+    const char* gen_why = gen_config_for(r_id, r_y, r_p, r_r, pl->gen);
+    pl->gen_ok = gen_why == nullptr;
     if (pl->nBCD > kMaxBCD && !pl->gen_ok) {
-        return set_error(NLML_E_UNSUPPORTED, "angle-mode ranks (%d,%d,%d) give %d folded entries per identity pair; limit %d "
-                         "(the tensor-core kernel for larger cores needs a roll rank <= 8)",
-                         r_y, r_p, r_r, tri(r_y) * tri(r_p) * tri(r_r), kMaxBCD);
+        return set_error(NLML_E_UNSUPPORTED, "angle-mode ranks (%d,%d,%d) give %d folded entries per identity pair, above the "
+                         "CTA-per-sample kernel's limit %d, and %s", r_y, r_p, r_r, pl->nBCD, kMaxBCD, gen_why);
     }
     cudaDeviceProp prop;
     NLML_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -2507,6 +2533,19 @@ extern "C" int nlml_tucker_powell_landmarks_f64(nlml_tucker_plan* pl, const floa
     return powell_launch(pl, LM_dev, N, ldx, 1, P_out_dev, ldp, fun_out_dev, nfev_out_dev, stream, nullptr, 0, nullptr);
 }
 /* test hook: q = W2 x of the tensor-core projection GEMM for N >= 4096 samples, CTA-blocked: Q_out_dev [ceil(N/128)][136][128] */
+extern "C" int nlml_debug_gen_config(int r_id, int r_y, int r_p, int r_r, int32_t* out, int n_out) {
+    constexpr int kFields = 23;
+    if (!out || n_out < kFields) return set_error(NLML_E_INVALID, "out needs room for %d fields", kFields);
+    if (r_id < 1 || r_y < 1 || r_p < 1 || r_r < 1) return set_error(NLML_E_INVALID, "ranks must be positive");
+    tgen::GenCfg c{};
+    if (const char* why = gen_config_for(r_id, r_y, r_p, r_r, c)) return set_error(NLML_E_UNSUPPORTED, "%s", why);
+    const int32_t v[kFields] = {c.rrmax, c.nA, c.KA, c.NA16, c.nBC, c.nDp, c.BCP, c.NB, c.nblocks, c.resident, c.tslots,
+                                c.gslots, c.ypr_tmem, c.tbufs, c.gbufs, c.ybufs, c.col_g, c.col_a, c.col_t, c.col_y,
+                                c.smem_bytes, c.tt_bytes, c.gt_bytes};
+    std::memcpy(out, v, sizeof(v));
+    return 0;
+}
+
 extern "C" int nlml_debug_project_tc(nlml_tucker_plan* pl, const float* X_dev, int64_t N, int64_t ldx, float* Q_out_dev) {
     if (!pl || !X_dev || !Q_out_dev) return set_error(NLML_E_INVALID, "null pointer argument");
     DeviceGuard guard(pl->device);

@@ -62,57 +62,59 @@ def sgd_reference_form(W, x, rows_y, rows_p, rows_r, lr=0.001, iters=3000, clip=
     return p.detach().numpy().copy()
 
 
-def _features_and_derivs(w, rows):
-    """w f32 [N]; rows f32 [R,4] -> (c, dc) f32 [N,R] each."""
+def _features_and_derivs(w, rows, dtype=np.float32):
+    """w [N]; rows [R,4] -> (c, dc) [N,R] each, in dtype."""
     a, b, c, d = rows[:, 0], rows[:, 1], rows[:, 2], rows[:, 3]
     arg = b[None, :] * w[:, None] + c[None, :]
     val = a[None, :] * np.cos(arg) + d[None, :]
     der = -(a * b)[None, :] * np.sin(arg)
-    return val.astype(np.float32), der.astype(np.float32)
+    return val.astype(dtype), der.astype(dtype)
 
 
-def gradient_batched(P, W, X, rows_y, rows_p, rows_r):
-    """Gradient of `objective` w.r.t. p for a batch, float32, direct (residual) form.
+def gradient_batched(P, W, X, rows_y, rows_p, rows_r, dtype=np.float32):
+    """Gradient of `objective` w.r.t. p for a batch, direct (residual) form, computed in dtype (float32: the
+    reference's arithmetic; float64: a check on how well a float32 result is conditioned).
 
     r = x_hat - x ; dL/dz = W2 r ; chain rule through z = u (x) c_y (x) c_p (x) c_r.
-    P f32 [N,3+R_id], X f32 [N,F] -> G f32 [N,3+R_id], loss f32 [N].
+    P [N,3+R_id], X [N,F] -> G [N,3+R_id], loss [N], both dtype.
     """
-    W = np.asarray(W, dtype=np.float32)
+    W = np.asarray(W, dtype=dtype)
     r_id, r_y, r_p, r_r, F = W.shape
     W2 = W.reshape(-1, F)
-    rows_y, rows_p, rows_r = (np.asarray(r, dtype=np.float32) for r in (rows_y, rows_p, rows_r))
-    P = np.asarray(P, dtype=np.float32)
-    cy, dcy = _features_and_derivs(P[:, 0], rows_y)
-    cp, dcp = _features_and_derivs(P[:, 1], rows_p)
-    cr, dcr = _features_and_derivs(P[:, 2], rows_r)
+    X = np.asarray(X, dtype=dtype)
+    rows_y, rows_p, rows_r = (np.asarray(r, dtype=dtype) for r in (rows_y, rows_p, rows_r))
+    P = np.asarray(P, dtype=dtype)
+    cy, dcy = _features_and_derivs(P[:, 0], rows_y, dtype)
+    cp, dcp = _features_and_derivs(P[:, 1], rows_p, dtype)
+    cr, dcr = _features_and_derivs(P[:, 2], rows_r, dtype)
     u = P[:, 3:]
-    z = np.einsum("ni,nj,nk,nl->nijkl", u, cy, cp, cr).reshape(len(P), -1).astype(np.float32)
+    z = np.einsum("ni,nj,nk,nl->nijkl", u, cy, cp, cr).reshape(len(P), -1).astype(dtype)
     res = z @ W2 - X
-    gz = (res @ W2.T).reshape(len(P), r_id, r_y, r_p, r_r).astype(np.float32)
+    gz = (res @ W2.T).reshape(len(P), r_id, r_y, r_p, r_r).astype(dtype)
     G = np.empty_like(P)
     G[:, 0] = np.einsum("nijkl,ni,nj,nk,nl->n", gz, u, dcy, cp, cr)
     G[:, 1] = np.einsum("nijkl,ni,nj,nk,nl->n", gz, u, cy, dcp, cr)
     G[:, 2] = np.einsum("nijkl,ni,nj,nk,nl->n", gz, u, cy, cp, dcr)
     G[:, 3:] = np.einsum("nijkl,nj,nk,nl->ni", gz, cy, cp, cr)
-    return G.astype(np.float32), (0.5 * (res * res).sum(1)).astype(np.float32)
+    return G.astype(dtype), (0.5 * (res * res).sum(1)).astype(dtype)
 
 
-def sgd_batched(W, X, rows_y, rows_p, rows_r, lr=0.001, iters=3000, clip=1.0, P0=None):
-    """Batched float32 restatement of TD_Tester.py:127-159 with the hand-written gradient.
+def sgd_batched(W, X, rows_y, rows_p, rows_r, lr=0.001, iters=3000, clip=1.0, P0=None, dtype=np.float32):
+    """Batched restatement of TD_Tester.py:127-159 with the hand-written gradient, in dtype (float32 = the reference).
 
     clip_grad_norm_ semantics (:150): g *= min(1, clip / (||g||_2 + 1e-6)), norm over all
-    3+R_id components jointly; update (:153-154): p -= lr * g.  Returns P f32 [N,3+R_id].
+    3+R_id components jointly; update (:153-154): p -= lr * g.  Returns P [N,3+R_id] in dtype.
     """
-    X = np.asarray(X, dtype=np.float32)
+    X = np.asarray(X, dtype=dtype)
     n = X.shape[0]
-    P = np.zeros((n, 3 + W.shape[0]), dtype=np.float32) if P0 is None else np.array(P0, dtype=np.float32)
-    lr32, clip32, eps32 = np.float32(lr), np.float32(clip), np.float32(1e-6)
+    P = np.zeros((n, 3 + W.shape[0]), dtype=dtype) if P0 is None else np.array(P0, dtype=dtype)
+    lr_, clip_, eps_ = dtype(lr), dtype(clip), dtype(1e-6)
     for _ in range(iters):
-        G, _ = gradient_batched(P, W, X, rows_y, rows_p, rows_r)
-        norm = np.sqrt((G * G).sum(1, dtype=np.float32)).astype(np.float32)
-        coef = np.minimum(clip32 / (norm + eps32), np.float32(1.0)).astype(np.float32)
-        G = (G * coef[:, None]).astype(np.float32)
-        P = (P - lr32 * G).astype(np.float32)
+        G, _ = gradient_batched(P, W, X, rows_y, rows_p, rows_r, dtype)
+        norm = np.sqrt((G * G).sum(1, dtype=dtype)).astype(dtype)
+        coef = np.minimum(clip_ / (norm + eps_), dtype(1.0)).astype(dtype)
+        G = (G * coef[:, None]).astype(dtype)
+        P = (P - lr_ * G).astype(dtype)
     return P
 
 
